@@ -28,6 +28,8 @@ config[2] (Llama-3-70B TP=8 per-rank shard, every rank concurrently, no collecti
   --incremental 1   sleeps whose weights still match the image in the host store release the device side without a copy
   --extras packed,incremental   (any N, opt-in) after the main line, on the same engines: bf16 refill, PACKED cycles, then
                     INCREMENTAL cycles, aggregated like the main line (reported under `extras`)
+  --dump-outputs DIR   after the timed steps, write what the last wake restored (every weight segment's digest and a fixed
+                    sample of the weight bytes) as DIR/*.npy, so that two builds can be compared output for output
 
 Synthetic data: counter-based splitmix64 bytes (seed 1234 + rank); the working set (>= 15 GiB per rank) is far
 larger than the 126 MB L2, so no L2 flush is needed between iterations.
@@ -208,6 +210,8 @@ def run_ours(args) -> None:
 
     after = eng.digest_all(["weights"])
     bit_exact = after == before
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, table, after, f"_rank{rank}" if world > 1 else "")
 
     mean = lambda xs: sum(xs) / len(xs)
     k2_s = sum(r[1]["kernel_seconds"] for r in rows); k2_b = sum(r[1]["kernel_bytes"] for r in rows)
@@ -335,6 +339,26 @@ def run_ours(args) -> None:
         print(json.dumps(out), flush=True)
     eng.close()
     group.close()
+
+
+def dump_outputs(out_dir: str, eng, table, digests: list[int], suffix: str, block: int = 4096, blocks: int = 2048) -> None:
+    """What the last timed wake handed back to its caller: the weight segments' contents.  weights_digest.npy holds the K3 digest
+    of every weight segment as (high, low) 32-bit halves in float64; weights_sample.npy holds the bytes of `blocks` 4 KiB blocks
+    drawn with a fixed seed from all weight segments, as float32 (32 MiB).  Both are the same from run to run unless a build
+    computes different bytes."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    idx = [i for i, s in enumerate(table) if s.tag == "weights"]
+    d = np.array([digests[i] for i in idx], dtype=np.uint64)
+    np.save(os.path.join(out_dir, f"weights_digest{suffix}.npy"), np.stack([d >> np.uint64(32), d & np.uint64(0xFFFFFFFF)], axis=1).astype(np.float64))
+    starts = np.cumsum([0] + [table[i].bytes // block for i in idx])        # first block of each weight segment
+    picks = np.sort(np.random.default_rng(0).choice(int(starts[-1]), size=min(blocks, int(starts[-1])), replace=False))
+    sample = np.empty((len(picks), block), dtype=np.float32)
+    for row, b in enumerate(picks):
+        k = int(np.searchsorted(starts, b, side="right")) - 1
+        sample[row] = np.frombuffer(eng.read(idx[k], block, offset=int(b - starts[k]) * block), dtype=np.uint8)
+    np.save(os.path.join(out_dir, f"weights_sample{suffix}.npy"), sample)
 
 
 def bench_config(args, workload: str, weight_bytes: int, n_segments: int, world: int, mode: str, packed: bool) -> dict:
@@ -934,6 +958,8 @@ def main() -> None:
     ap.add_argument("--scaling-workload", default="llama-3-70b-tp8", help="table of the scaling_base extra (= the N>1 workload)")
     ap.add_argument("--extras-kv-gib", type=float, default=16.0, help="kv_cache bytes per model in the swap / roundrobin extras")
     ap.add_argument("--timeline", default="", help="directory: every rank writes the per-phase timeline (fma_timeline) of its last timed sleep and wake there")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the weights the last wake restored (digests and a fixed sample) to DIR/*.npy")
     ap.add_argument("--packed-child", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.packed_child:

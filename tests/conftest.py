@@ -1,5 +1,7 @@
 import os
+import shutil
 import sys
+import tempfile
 
 import pytest
 
@@ -36,3 +38,12 @@ def engine(built):
     eng = fma_b200.Engine(0)
     yield eng
     eng.close()
+
+
+@pytest.fixture()
+def sock_dir():
+    """A directory for unix sockets.  An AF_UNIX path holds at most 107 bytes, which a socket under tmp_path exceeds when the
+    temporary directory has a long name, so the sockets go to a short directory under /tmp."""
+    d = tempfile.mkdtemp(prefix="fma-", dir="/tmp")
+    yield d
+    shutil.rmtree(d, ignore_errors=True)

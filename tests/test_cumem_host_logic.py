@@ -2,6 +2,7 @@
 reference's (cumem.py:186-194), tiers/knobs come from the environment, and the INFO line the reference's benchmark
 tooling parses (cumem.py:215-222; inference_server/benchmark/benchmark.md:157) keeps its wording."""
 import logging
+import os
 import re
 
 import pytest
@@ -94,7 +95,7 @@ def test_peer_tier_comes_from_the_environment(alloc, monkeypatch):
         alloc.sleep(offload_tags=("weights",))
 
 
-def test_peer_tier_falls_back_to_the_host_tier_when_no_gpu_can_take_the_image(alloc, monkeypatch, tmp_path, caplog):
+def test_peer_tier_falls_back_to_the_host_tier_when_no_gpu_can_take_the_image(alloc, monkeypatch, sock_dir, caplog):
     """Under the node agent the parking buffer is the agent's (parking.py).  If every candidate GPU is full — or the agent is gone —
     the sleep still has to succeed: it goes to the host tier, as the reference's always does (cumem.py:237-249), and says so."""
     from fma_b200.parking import ParkingService
@@ -102,7 +103,7 @@ def test_peer_tier_falls_back_to_the_host_tier_when_no_gpu_can_take_the_image(al
     def full(device, nbytes):
         raise MemoryError(f"cuMemCreate on device {device}: out of memory")
 
-    sock = str(tmp_path / "agent.sock")
+    sock = os.path.join(sock_dir, "agent.sock")
     svc = ParkingService(sock, n_devices=4, make_buffer=full)
     svc.start()
     monkeypatch.setenv("FMA_TIER", "peer")

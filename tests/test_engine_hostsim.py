@@ -138,16 +138,42 @@ print("ok")
 def test_bench_main_flow_runs_against_the_host_simulated_engine(hostsim_lib, oracle, tmp_path):
     """The whole of bench.py's own arm at N=1 — table, fill, digests, timed cycles, JSON line with every contract key,
     cpu_baseline fallback (the oracle port: vLLM's allocator cannot load here) and the packed_image child — with torch
-    replaced by tests/stubs/torch.  Numbers are meaningless here; the flow and the keys are what is checked."""
+    replaced by tests/stubs/torch.  Numbers are meaningless here; the flow and the keys are what is checked.  --dump-outputs
+    writes the restored weights (digests == the oracle's, a byte sample), and a second run with the same arguments writes the
+    same arrays."""
     import json
+
+    import numpy as np
 
     env = dict(os.environ, FMA_B200_LIB=hostsim_lib, FMA_HOSTSIM="1", HOSTSIM_DEVICES="2",
                PYTHONPATH=os.path.join(ROOT, "tests", "stubs") + os.pathsep + os.environ.get("PYTHONPATH", ""))
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny-llama-test", "--kv-gib", "0.03125",
                         "--steps", "2", "--warmup", "3", "--swap-models", "tiny-llama-test,tiny-llama-test", "--scaling-workload", "opt-125m",
-                        "--extras-kv-gib", "0.03125", "--timeline", str(tmp_path / "tl")], env=env, cwd=ROOT, capture_output=True, text=True, timeout=900)
+                        "--extras-kv-gib", "0.03125", "--timeline", str(tmp_path / "tl"), "--dump-outputs", str(tmp_path / "out")],
+                       env=env, cwd=ROOT, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, (r.stdout + r.stderr)[-3000:]
     out = json.loads(r.stdout.strip().splitlines()[-1])
+    assert out["steps"] == 2 and len(out["wake_latency_s_steps"]) == 2
+    r2 = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny-llama-test", "--kv-gib", "0.03125",
+                         "--steps", "1", "--warmup", "3", "--extras", "", "--packed-extra", "0", "--no-cpu-baseline",
+                         "--dump-outputs", str(tmp_path / "out2")], env=env, cwd=ROOT, capture_output=True, text=True, timeout=900)
+    assert r2.returncode == 0, (r2.stdout + r2.stderr)[-3000:]
+    assert json.loads(r2.stdout.strip().splitlines()[-1])["steps"] == 1
+    import fma_b200  # noqa: F401
+    from fma_b200 import workloads as W
+
+    weights = [s for s in W.allocation_table("tiny-llama-test") if s.tag == "weights"]
+    want, first = [], 0
+    for s in weights:
+        want.append(oracle.digest(oracle.fill(s.bytes, 1234, first)))
+        first += s.bytes // 8
+    for name in ("weights_digest", "weights_sample"):
+        a, b = np.load(tmp_path / "out" / f"{name}.npy"), np.load(tmp_path / "out2" / f"{name}.npy")
+        assert a.dtype in (np.float32, np.float64) and a.nbytes <= 64 << 20 and np.array_equal(a, b), name
+    dg = np.load(tmp_path / "out" / "weights_digest.npy")
+    assert [int(hi) << 32 | int(lo) for hi, lo in dg] == want
+    sample = np.load(tmp_path / "out" / "weights_sample.npy")
+    assert sample.shape == (2048, 4096) and sample.min() >= 0 and sample.max() <= 255 and sample.std() > 50
     assert out["swap_config4"].get("bit_exact") is True and out["swap_config4"]["cycles"] == 20, out["swap_config4"]
     assert out["n1_on_scaling_workload"].get("bit_exact") is True, out["n1_on_scaling_workload"]
     assert out["multipath_wake"].get("bit_exact") is True and out["multipath_wake"]["rows"][0]["paths"] == 2, out["multipath_wake"]
@@ -302,14 +328,14 @@ else:
 """
 
 
-def test_node_level_parking_service_keeps_a_dead_instances_image(hostsim_lib, tmp_path):
+def test_node_level_parking_service_keeps_a_dead_instances_image(hostsim_lib, tmp_path, sock_dir):
     """fma_b200.parking: the node agent's ParkingService owns exportable parking buffers and serves fds over a unix socket; an
     instance parks its weights there, deposits the descriptor and DIES; a fresh instance with the same ID finds the image, attaches,
     adopts and wakes with identical K3 digests; the owner's accounting (MiB per GPU — what a sleeper budget needs,
     inference-server.go:1609-1636) follows.  Host-simulated engine; the C-ABI underneath is GPU-tested in tests/test_gpu_parity.py."""
     import json
 
-    env = dict(os.environ, FMA_B200_LIB=hostsim_lib, FMA_HOSTSIM="1", HOSTSIM_DEVICES="3", FMA_NODE_AGENT_SOCK=str(tmp_path / "park.sock"))
+    env = dict(os.environ, FMA_B200_LIB=hostsim_lib, FMA_HOSTSIM="1", HOSTSIM_DEVICES="3", FMA_NODE_AGENT_SOCK=os.path.join(sock_dir, "park.sock"))
     owner = r"""
 import os, sys, json, subprocess
 sys.path.insert(0, %r)

@@ -1,7 +1,8 @@
-"""Differential test of the node agent against the LIVE, UNMODIFIED reference launcher (baseline/_ref, staged by build()):
-the same request script runs against both services on CPU (children = the config-0 stand-in) and every status code,
-header of interest and JSON shape must agree.  Then the node-scoped routes the reference does not have
-(sleep / wake_up / is_sleeping proxies, swap, sleepers) are exercised on the agent."""
+"""Differential test of the node agent against the UNMODIFIED reference launcher: the same request script runs on CPU
+(children = the config-0 stand-in) and every status code, header of interest and JSON shape must agree with what the
+reference launcher answered to it (tests/golden/launcher_rest.json, written by tests/golden/make_launcher_golden.py).
+Then the node-scoped routes the reference does not have (sleep / wake_up / is_sleeping proxies, swap, sleepers) are
+exercised on the agent."""
 import json
 import os
 import socket
@@ -14,7 +15,7 @@ import urllib.request
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LAUNCHER = os.path.join(ROOT, "baseline", "_ref", "launcher", "launcher.py")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "launcher_rest.json")
 AGENT = os.path.join(ROOT, "scripts", "run_node_agent.py")
 ENV_PATH = os.pathsep.join([os.path.join(ROOT, "scripts", "vllm_cpu_standin"), os.path.join(ROOT, "scripts", "k8s_stub"), ROOT])
 
@@ -50,16 +51,18 @@ def _wait(url, seconds=60):
 
 
 class Service:
-    def __init__(self, kind, tmp_path):
-        self.kind, self.port = kind, _port()
+    """A launcher-compatible REST service (the node agent, or the reference launcher when the golden file is written)."""
+
+    def __init__(self, script, log_dir):
+        self.port = _port()
         env = dict(os.environ)
         env["PYTHONPATH"] = os.pathsep.join([ENV_PATH, env.get("PYTHONPATH", "")])
-        script = LAUNCHER if kind == "reference" else AGENT
-        self.log = open(tmp_path / f"{kind}.log", "w")
+        log = os.path.join(log_dir, "service.log")
+        self.log = open(log, "w")
         self.proc = subprocess.Popen([sys.executable, script, "--mock-gpus", "--host", "127.0.0.1", "--port", str(self.port)],
                                      env=env, cwd=os.path.dirname(script), stdout=self.log, stderr=subprocess.STDOUT)
         self.base = f"http://127.0.0.1:{self.port}"
-        assert _wait(self.base + "/health"), open(tmp_path / f"{kind}.log").read()[-2000:]
+        assert _wait(self.base + "/health"), open(log).read()[-2000:]
 
     def close(self):
         self.proc.terminate()
@@ -70,12 +73,20 @@ class Service:
 
 
 @pytest.fixture()
-def both(built, tmp_path):
-    if not os.path.exists(LAUNCHER):
-        pytest.skip("reference launcher not staged (no /root/reference at build time)")
-    ref, mine = Service("reference", tmp_path), Service("agent", tmp_path)
-    yield ref, mine
-    ref.close(); mine.close()
+def mine(built, tmp_path):
+    svc = Service(AGENT, str(tmp_path))
+    yield svc
+    svc.close()
+
+
+def _reference(key):
+    """What the reference launcher answered to the same script (JSON: tuples are stored as lists)."""
+    with open(GOLDEN) as f:
+        return json.load(f)[key]
+
+
+def _as_stored(x):
+    return json.loads(json.dumps(x))
 
 
 def _shape(x):
@@ -150,10 +161,9 @@ def _script(svc, vport):
     return obs
 
 
-def test_same_rest_contract_as_the_reference_launcher(both):
-    ref, mine = both
-    a = _script(ref, _port())
-    b = _script(mine, _port())
+def test_same_rest_contract_as_the_reference_launcher(mine):
+    a = _reference("rest_contract")
+    b = _as_stored(_script(mine, _port()))
     assert [x[0] for x in a] == [x[0] for x in b]
     for ra, rb in zip(a, b):
         assert ra == rb, f"{ra[0]}: reference {ra[1:]} != agent {rb[1:]}"
@@ -170,47 +180,51 @@ def _read_events(url, n, timeout=20):
     return out
 
 
-def test_watch_stream_matches_the_reference(both):
-    seqs = []
-    for svc in both:
-        vport = _port()
-        cfg = {"options": f"--port {vport} --host 127.0.0.1", "annotations": {"inference-port": str(vport)}}
-        assert _http("PUT", svc.base + "/v2/vllm/instances/w1", cfg)[0] == 201
-        import threading
+def _watch_script(svc):
+    vport = _port()
+    cfg = {"options": f"--port {vport} --host 127.0.0.1", "annotations": {"inference-port": str(vport)}}
+    assert _http("PUT", svc.base + "/v2/vllm/instances/w1", cfg)[0] == 201
+    import threading
 
-        got = []
-        t = threading.Thread(target=lambda: got.extend(_read_events(svc.base + "/v2/vllm/instances/watch", 3)))
-        t.start(); time.sleep(1.0)                                           # watcher connected: gets CREATED(w1) first
-        assert _http("PUT", svc.base + "/v2/vllm/instances/w2", {"options": f"--port {_port()} --host 127.0.0.1"})[0] == 201
-        assert _http("DELETE", svc.base + "/v2/vllm/instances/w2")[0] == 200
-        t.join(timeout=30)
-        seqs.append([(e["type"], e["object"]["instance_id"], e["object"]["status"], sorted(e["object"])) for e in got])
-        # resume from revision 1: only what happened after the first create
-        later = _read_events(svc.base + "/v2/vllm/instances/watch?since=1", 2)
-        seqs[-1].append([(e["type"], e["object"]["instance_id"], e["object"]["revision"]) for e in later])
-        _http("DELETE", svc.base + "/v2/vllm/instances")
-    assert seqs[0] == seqs[1]
-    assert [e[0] for e in seqs[1][:3]] == ["CREATED", "CREATED", "DELETED"]
+    got = []
+    t = threading.Thread(target=lambda: got.extend(_read_events(svc.base + "/v2/vllm/instances/watch", 3)))
+    t.start(); time.sleep(1.0)                                           # watcher connected: gets CREATED(w1) first
+    assert _http("PUT", svc.base + "/v2/vllm/instances/w2", {"options": f"--port {_port()} --host 127.0.0.1"})[0] == 201
+    assert _http("DELETE", svc.base + "/v2/vllm/instances/w2")[0] == 200
+    t.join(timeout=30)
+    seq = [(e["type"], e["object"]["instance_id"], e["object"]["status"], sorted(e["object"])) for e in got]
+    # resume from revision 1: only what happened after the first create
+    later = _read_events(svc.base + "/v2/vllm/instances/watch?since=1", 2)
+    seq.append([(e["type"], e["object"]["instance_id"], e["object"]["revision"]) for e in later])
+    _http("DELETE", svc.base + "/v2/vllm/instances")
+    return seq
 
 
-def test_stopped_event_when_a_child_dies(both):
+def test_watch_stream_matches_the_reference(mine):
+    seq = _as_stored(_watch_script(mine))
+    assert _reference("watch") == seq
+    assert [e[0] for e in seq[:3]] == ["CREATED", "CREATED", "DELETED"]
+
+
+def _child_dies_script(svc):
+    vport = _port()
+    assert _http("PUT", svc.base + "/v2/vllm/instances/dies", {"options": f"--port {vport} --host 127.0.0.1"})[0] == 201
+    assert _wait(f"http://127.0.0.1:{vport}/health")
+    psutil = pytest.importorskip("psutil")
+    pid = next((c.pid for c in psutil.net_connections(kind="tcp") if c.laddr and c.laddr.port == vport and c.status == "LISTEN" and c.pid), None)
+    if pid is None:
+        pytest.skip("cannot find the child's pid")
+    os.kill(pid, 9)
+    ev = _read_events(svc.base + "/v2/vllm/instances/watch?since=1", 1)
+    st = json.loads(_http("GET", svc.base + "/v2/vllm/instances/dies")[1])
+    _http("DELETE", svc.base + "/v2/vllm/instances")
+    return (ev[0]["type"], ev[0]["object"]["status"], ev[0]["object"]["exit_code"], st["status"], sorted(ev[0]["object"]))
+
+
+def test_stopped_event_when_a_child_dies(mine):
     """A child that exits by itself is reported as STOPPED with its exit code, and stays listed as 'stopped'."""
-    outs = []
-    for svc in both:
-        vport = _port()
-        assert _http("PUT", svc.base + "/v2/vllm/instances/dies", {"options": f"--port {vport} --host 127.0.0.1"})[0] == 201
-        assert _wait(f"http://127.0.0.1:{vport}/health")
-        psutil = pytest.importorskip("psutil")
-        pid = next((c.pid for c in psutil.net_connections(kind="tcp") if c.laddr and c.laddr.port == vport and c.status == "LISTEN" and c.pid), None)
-        if pid is None:
-            pytest.skip("cannot find the child's pid")
-        os.kill(pid, 9)
-        ev = _read_events(svc.base + "/v2/vllm/instances/watch?since=1", 1)
-        st = json.loads(_http("GET", svc.base + "/v2/vllm/instances/dies")[1])
-        outs.append((ev[0]["type"], ev[0]["object"]["status"], ev[0]["object"]["exit_code"], st["status"], sorted(ev[0]["object"])))
-        _http("DELETE", svc.base + "/v2/vllm/instances")
-    ref, mine = outs
-    assert mine[:4] == ("STOPPED", "stopped", -9, "stopped")
+    ref, mine = _reference("child_dies"), _as_stored(_child_dies_script(mine))
+    assert mine[:4] == ["STOPPED", "stopped", -9, "stopped"]
     # same event type, same keys, same final listing.  The reference's event body is racy here: its exit watcher fires
     # when the child's sentinel pipe closes, which the kernel does BEFORE the process becomes reapable, so
     # `is_alive()`/`exitcode` inside the callback can still say running/None (launcher.py:256-266,372-382).
@@ -218,8 +232,7 @@ def test_stopped_event_when_a_child_dies(both):
     assert (ref[1], ref[2]) in {("stopped", -9), ("running", None)}
 
 
-def test_node_scoped_actuation_routes(both):
-    _, mine = both
+def test_node_scoped_actuation_routes(mine):
     pa, pb = _port(), _port()
     for iid, p in (("model-a", pa), ("model-b", pb)):
         cfg = {"options": f"--enable-sleep-mode --port {p} --host 127.0.0.1", "env_vars": {"VLLM_SERVER_DEV_MODE": "1"},

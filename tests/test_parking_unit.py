@@ -44,12 +44,12 @@ class FakeEngine:
         self.adopted = (desc, tuple(tags))
 
 
-def test_placement_accounting_and_protocol(tmp_path):
+def test_placement_accounting_and_protocol(sock_dir):
     FakeBuffer.made.clear()
-    svc = ParkingService(str(tmp_path / "s.sock"), n_devices=4, make_buffer=FakeBuffer)
+    svc = ParkingService(os.path.join(sock_dir, "s.sock"), n_devices=4, make_buffer=FakeBuffer)
     svc.start()
     try:
-        cli = ParkingClient(str(tmp_path / "s.sock"))
+        cli = ParkingClient(os.path.join(sock_dir, "s.sock"))
         e = FakeEngine()
         r = cli.park(e, "Ia", 0, 100 * MiB, avoid=[0])
         assert r["device"] == 1 and e.attached == 100 * MiB                    # least-loaded GPU outside `avoid`, lowest index first
